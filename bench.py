@@ -241,7 +241,7 @@ def run_b200(args):
     if os.environ.get("TB200_STEP_PARALLEL_MIN_MB"):  # experiment knob (see include/tb200.h)
         _native.check(_native.load().tb200_tune(b"step_parallel_min_mb", int(os.environ["TB200_STEP_PARALLEL_MIN_MB"])))
     # --- e2e: the same step through the public API, job tables H2D + results D2H every step
-    e2e_steps = max(10, min(steps, 20000))
+    e2e_steps = steps
     for i in range(warmup):
         ops.fill(fill_jobs[i % SETS], seed=SEED, epoch=i * SLOTS)
         ops.check(check_jobs[i % SETS], results.device_ptr + (i % SETS) * SLOTS * 32)
@@ -287,6 +287,15 @@ def run_b200(args):
     e2e_ms = rep.max(max(timer.elapsed_ms(), e2e_wall_ms))
     assert bad == 0
     assert SETS > E2E_DEPTH  # steps in flight use different slot sets and result entries
+    # what the last of these steps handed its caller: the 64 generated inputs and the 64 verdicts.
+    # This loop, not the loopback generator, is dumped because its epochs depend only on the step
+    # index; the generator batches requests into device passes as they happen to arrive.
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        s = (e2e_steps - 1) % SETS
+        last = res[s * SLOTS:(s + 1) * SLOTS]
+        outputs = {"inputs": ops.download(in_regions[s]._base_addr, SLOTS * IN_BYTES, np.float32).reshape((SLOTS,) + IN_SHAPE)}
+        outputs.update({"check_" + f: last[f].astype(np.float64) for f in ("mismatches", "sum", "xor32", "argmax", "max_value")})
     api_value = world * SLOTS * e2e_steps / (e2e_ms / 1e3)
     h2d_step = SLOTS * 64 + (SLOTS + 1) * 4 + SLOTS * 48
     d2h_step = SLOTS * 32
@@ -559,6 +568,10 @@ def run_b200(args):
             line["wire_c4_c5"] = wire_extra(ops, ctx, local)
         except Exception as ex:
             line["wire_c4_c5"] = {"error": "%s: %s" % (type(ex).__name__, ex)}
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if rank == 0:
         print(json.dumps(line), flush=True)
     rep.close()
@@ -961,13 +974,27 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20000)
+    ap.add_argument("--steps", type=int, default=20000,
+                    help="timed steps of each repetition of the headline generator and of the DeviceOps step_submit/step_wait "
+                         "loop (the one --dump-outputs writes).  Sections that need a longer or shorter window derive "
+                         "their own count from it, each reported in the JSON line: the generator-capacity graphs run at "
+                         "least 8000 steps, the synchronous API loop a quarter of --steps but at least 10, the host-image "
+                         "loop 5 to 2000, the time-sliced run at most 2000")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-loopback", action="store_true", help="skip the extra loopback levels (other concurrencies, gRPC configs, the run without MPS)")
     ap.add_argument("--no-mps", action="store_true", help="do not start a CUDA MPS daemon: client and server time-slice the GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed DeviceOps step returned to DIR (rank 0 only): inputs.npy, the 64 "
+                         "FP32[3,224,224] tensors the fill kernel generated for that step; check_<field>.npy, the validate "
+                         "kernel's 64 results (float64) over the response logits, which are written once at setup and so "
+                         "are the same for every step and every --steps")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

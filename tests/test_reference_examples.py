@@ -1,7 +1,8 @@
 """The reference's own example scripts, UNMODIFIED, run against the drop-in package
 (`client_b200.install_as_tritonclient()`) and the mock server: every script ends with its own
 value checks and exits non-zero on a mismatch (SURVEY.md section 4, "examples as tests").
-Needs /root/reference (present in the build container, absent on the GPU box -> skipped there).
+The Python example scripts are read from the reference's source tree; where it is absent those
+tests skip.  The C++ programs run from the binaries build() compiled under oracle/_ref/cc_examples/.
 Not run: the CUDA shared memory examples (GPU tests restate them), the model-control examples
 (server repository semantics), simple_http_infer_client.py (imports gevent itself, absent here),
 ensemble_image_client.py / image_client.py over HTTP (import attrdict, absent here)."""
@@ -39,7 +40,8 @@ IMAGE_RUNS = [
     ("grpc_image_client.py", ["-m", "densenet_onnx", "-s", "INCEPTION", "-c", "3"]),
 ]
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(EXAMPLES), reason="the reference tree is not mounted")
+# the scripts are the reference's own sources, which the repository does not carry
+needs_reference = pytest.mark.skipif(not os.path.isdir(EXAMPLES), reason="the reference's Python examples are absent")
 
 
 @pytest.fixture(scope="module")
@@ -79,6 +81,7 @@ def outcomes(tmp_path_factory):
     return results
 
 
+@needs_reference
 @pytest.mark.parametrize("label", SCRIPTS + ["%s %s" % (n, " ".join(a)) for n, a in IMAGE_RUNS])
 def test_unmodified_reference_example(outcomes, label):
     rc, tail = outcomes[label]
@@ -115,6 +118,7 @@ def native_transport_outcomes(tmp_path_factory):
         proc.wait(10)
 
 
+@needs_reference
 @pytest.mark.parametrize("name", NATIVE_TRANSPORT_SCRIPTS)
 def test_unmodified_reference_example_on_the_native_grpc_transport(native_transport_outcomes, name):
     """The examples whose inferences are synchronous infer() calls, run with the drop-in's native
@@ -151,9 +155,20 @@ CC_EXAMPLES = {
 
 @pytest.fixture(scope="module")
 def cc_binaries():
+    """{name: path}: built from the reference's sources where they are present, otherwise the
+    binaries an earlier build() left under oracle/_ref/cc_examples/ (they travel with the tree)."""
     from oracle.build_ref_examples import build_ref_examples
 
-    return build_ref_examples()
+    built = build_ref_examples()
+    if not built and os.path.isdir(CC_OUT):
+        built = {f: os.path.join(CC_OUT, f) for f in os.listdir(CC_OUT) if os.access(os.path.join(CC_OUT, f), os.X_OK)}
+    return built
+
+
+def _cc_binary(cc_binaries, name):
+    if name not in cc_binaries:
+        pytest.skip("oracle/_ref/cc_examples/%s was not built: no reference source tree at build time" % name)
+    return cc_binaries[name]
 
 
 @pytest.fixture(scope="module")
@@ -170,10 +185,10 @@ def test_unmodified_reference_cc_example(cc_binaries, cc_server, name):
     libtb200client.so (oracle/build_ref_examples.py) and run against the mock server's models;
     the programs end with their own value checks."""
     exe, _, variant = name.partition(":")
-    assert exe in cc_binaries
+    path = _cc_binary(cc_binaries, exe)
     grpc = "_grpc_" in exe or variant == "grpc"
     url = cc_server["grpc" if grpc else "http"]
-    r = subprocess.run([cc_binaries[exe], "-u", url] + (["-i", "grpc"] if variant == "grpc" else []), capture_output=True, text=True, timeout=60)
+    r = subprocess.run([path, "-u", url] + (["-i", "grpc"] if variant == "grpc" else []), capture_output=True, text=True, timeout=60)
     assert r.returncode == 0 and CC_EXAMPLES[name] in r.stdout + r.stderr, r.stdout[-800:] + r.stderr[-400:]
 
 
@@ -182,8 +197,7 @@ def test_reference_client_timeout_test_unmodified(cc_binaries):
     is): sync / async / streaming over gRPC and sync / async over HTTP succeed with a generous
     client time-out and fail with the reference's "Deadline Exceeded" when the model takes 300 ms
     and the client allows 50 ms."""
-    exe = cc_binaries.get("client_timeout_test")
-    assert exe
+    exe = _cc_binary(cc_binaries, "client_timeout_test")
     modes = (["-i", "grpc"], ["-i", "grpc", "-a"], ["-i", "grpc", "-s"], ["-i", "http"], ["-i", "http", "-a"])
     for extra, timeout_us, rc in (((), "5000000", 0), (("--delay-us", "300000"), "50000", 1)):
         proc, http_port, grpc_port = start_server(extra)
@@ -203,8 +217,7 @@ def test_reference_memory_leak_test_unmodified(cc_binaries, cc_server):
     """src/c++/tests/memory_leak_test.cc (compiled as is; the reference runs it under valgrind):
     200 vs 2000 repetitions, new client per repetition and one reused client, over HTTP and gRPC --
     the peak resident set must not grow with the repetition count."""
-    exe = cc_binaries.get("memory_leak_test")
-    assert exe
+    exe = _cc_binary(cc_binaries, "memory_leak_test")
 
     def peak_kb(args):
         code = ("import resource, subprocess, sys; r = subprocess.run(%r, capture_output=True); "
@@ -221,12 +234,11 @@ def test_reference_memory_leak_test_unmodified(cc_binaries, cc_server):
 
 
 def test_reference_unit_tests_for_system_shared_memory_unmodified():
-    """src/python/library/tests/test_shared_memory.py (the reference's own unittest module)
-    loaded as is with the drop-in aliased as `tritonclient`."""
-    runner = ("import sys, unittest, importlib.util; sys.path.insert(0, %r); import client_b200; client_b200.install_as_tritonclient(); "
-              "spec = importlib.util.spec_from_file_location('ref_shm_tests', '/root/reference/src/python/library/tests/test_shared_memory.py'); "
-              "mod = importlib.util.module_from_spec(spec); spec.loader.exec_module(mod); "
-              "res = unittest.TextTestRunner(verbosity=0).run(unittest.TestLoader().loadTestsFromModule(mod)); "
-              "print('RAN', res.testsRun, len(res.failures), len(res.errors)); sys.exit(0 if res.wasSuccessful() else 1)" % ROOT)
-    r = subprocess.run([sys.executable, "-W", "ignore", "-c", runner], capture_output=True, text=True, timeout=120)
+    """src/python/library/tests/test_shared_memory.py (the reference's own unittest module, carried
+    byte for byte as tests/golden/reference_tests/test_shared_memory.py) loaded as is with the
+    drop-in aliased as `tritonclient`: the same run as
+    test_reference_unit_tests.py::test_reference_system_shared_memory_unit_tests_unmodified."""
+    from test_reference_unit_tests import _run
+
+    r = _run("test_shared_memory.py", timeout=120)
     assert r.returncode == 0 and "RAN 7 0 0" in r.stdout, r.stdout + r.stderr
